@@ -14,6 +14,10 @@ The K timed steps are taken at schedule positions spread evenly over the samplin
 of a run (self-attention injection on for t > (1 - inject_selfattn) * 1000, off afterwards) are timed in the proportion
 a full sampling run has them. Every CUDA-graph / exchange / cuDNN-autotune state the timed steps can reach is
 executed once before the timed region.
+
+`--dump-outputs DIR` writes what the last timed step returned (latents; SDXL configs also the guided noise prediction
+and the colour loss) as DIR/<name>.npy in float32. Weights and inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -155,6 +159,14 @@ def ncu_traffic(kernel_key):
         d = json.load(f)
     e = d.get(kernel_key)
     return (e["bytes_per_launch"], e["note"]) if e else (None, None)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every tensor of `arrays` as out_dir/<name>.npy, float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def host_threads():
@@ -390,6 +402,16 @@ def run_product_xl(args, rank, world, local_rank):
         ms = e0.elapsed_time(e1)
         launches = ops.LAUNCHES - launches0
         clk = clocks.stop() if clocks else None
+    if args.dump_outputs:   # the last timed step's result, written once per image by the lowest rank that holds it
+        out = {}
+        for im, st in zip(my_images, states):
+            holders = [r for r in range(world) if cfg["images"] == 1 or im in image_groups(world, r, cfg["images"])[0]]
+            if rank == holders[0]:
+                pre = f"image{im}_" if cfg["images"] > 1 else ""
+                out[pre + "latents"], out[pre + "noise_pred"] = st.latents, st.noise_pred
+        if rank == 0 and "color_loss" in model.last_step_stats:
+            out["color_loss"] = model.last_step_stats["color_loss"]
+        dump_outputs(args.dump_outputs, out)
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -655,6 +677,8 @@ def run_product_sd(args, rank, world, local_rank):
         launches = ops.LAUNCHES - launches0
         clk = clocks.stop() if clocks else None
         assert bool(torch.isfinite(out.float()).all())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"latents": out})
         host_lat = torch.empty(1, 4, 64, 64, dtype=torch.float16).pin_memory()
         barrier()
         t0 = time.perf_counter()
@@ -712,7 +736,12 @@ def main():
     ap.add_argument("--impl", default="rtti", choices=["rtti", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--check", action="store_true", help="N > 1: also compare with a single-GPU run of the same steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the product arm (--impl rtti)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -8,6 +8,7 @@ path (tests/test_parity_gpu.py, GPU). Weights are never stored: both sides rebui
 oracle.unet_oracle.make_state_dict(cfg, seed). The two schedulers are the restated third-party ones
 (oracle/schedulers_oracle.py) on both arms — diffusers is not installed.
 """
+import json
 import os
 import sys
 import types
@@ -323,10 +324,77 @@ def gen_token_maps(ns):
     print("token maps ok", [float(x.mean()) for x in masks])
 
 
+def gen_oracle_vs_reference(ns):
+    """Reference outputs on the inputs tests/test_oracle_vs_reference.py defines: UNet outputs and parameter
+    inventories, one font-size attention call, the text preparation of the Quill deltas, XL rich-text loops."""
+    from tests import test_oracle_vs_reference as t
+    res = {}
+
+    def inventory(name, model):
+        sd = model.state_dict()
+        res[f"{name}_names"] = np.array(list(sd))
+        res[f"{name}_shapes"] = np.array([",".join(str(d) for d in v.shape) for v in sd.values()])
+
+    for cfg_fn, seed in t.UNET_CASES:
+        cfg = cfg_fn()
+        model = ns.unet_2d_condition.UNet2DConditionModel(**cfg.ref_kwargs())
+        model.load_state_dict(uo.make_state_dict(cfg, seed))
+        inventory(cfg_fn.__name__, model)
+        x, ctx, added = t.unet_inputs(cfg, seed)
+        with torch.no_grad(), t.one_thread():
+            for i, ts in enumerate(t.UNET_TIMESTEPS):
+                res[f"{cfg_fn.__name__}_out{i}"] = model(x, ts, encoder_hidden_states=ctx, added_cond_kwargs=added)["sample"].numpy()
+    for cfg_fn in (uo.sd15_config, uo.sdxl_config):
+        with torch.device("meta"):
+            inventory(cfg_fn.__name__, ns.unet_2d_condition.UNet2DConditionModel(**cfg_fn().ref_kwargs()))
+
+    attn = ns.attention_processor.Attention(query_dim=64, cross_attention_dim=48, heads=2, dim_head=32)
+    sd, hs, ctx, aw = t.attention_inputs()
+    attn.load_state_dict({k[len("a."):]: v for k, v in sd.items()})
+    with torch.no_grad():
+        o, (pavg, p) = attn(hs, None, aw, encoder_hidden_states=ctx)
+    res.update(attn_out=o.numpy(), attn_pavg=pavg.numpy(), attn_probs=p.numpy())
+
+    rr = ns.richtext_utils
+    records = []
+    for delta in t._DELTAS:
+        out = rr.parse_json(delta)
+        base, styles, notes, note_t, cspans, cnames, crgbs, sizes, use_grad = out
+        rdi = rr.get_region_diffusion_input(t._Model(), base, styles, notes, note_t, cspans, cnames)
+        aci = rr.get_attention_control_input(t._Model(), rdi[2], sizes)
+        ggi = rr.get_gradient_guidance_input(t._Model(), rdi[2], cspans, crgbs, dict(aci), color_guidance_weight=0.5)
+        records.append({"delta": delta, "parse_json": t.to_json(out), "region_diffusion_input": t.to_json(rdi),
+                        "attention_control_input": t.to_json(aci), "gradient_guidance_input": t.to_json(ggi)})
+    with open(os.path.join(GOLD, "richtext_reference.json"), "w") as f:
+        json.dump(records, f, indent=1)
+        f.write("\n")
+
+    if ns.region_diffusion_sdxl is None:
+        raise RuntimeError(ns.region_diffusion_sdxl_error)
+    cfg = uo.tiny_xl_config()
+    S = 128
+    for case, (n_prompts, steps, inject_selfattn, inject_background, use_guidance, with_fs, seed) in enumerate(t.XL_CASES):
+        inp = synth_inputs(cfg, n_prompts, S, seed)
+        ctx, te = inp["ctx"], inp["text_embeds"]
+        m = make_xl_sampler(ns, cfg, 5, (ctx[1:], ctx[:1], te[1:], te[:1]))
+        m.masks = inp["masks"]
+        tfd = text_format(1, S, seed, with_fs=with_fs)
+        if use_guidance:
+            tfd.update(color_dict(inp["masks"], S, weight=0.7))
+        out = m.sample(["p"] * n_prompts, height=S * 8, width=S * 8, num_inference_steps=steps, guidance_scale=6.0,
+                       negative_prompt=[""], latents=inp["latents"].clone(), output_type="latent", use_guidance=use_guidance,
+                       inject_selfattn=inject_selfattn, inject_background=inject_background, text_format_dict=dict(tfd),
+                       run_rich_text=True).images.detach()
+        assert out.shape == (1, 4, S, S) and torch.isfinite(out).all()
+        res[f"xl{case}_latents_sample"] = out.flatten().numpy()[t.xl_sample_index()]
+    np.savez_compressed(os.path.join(GOLD, "oracle_vs_reference.npz"), **res)
+    print("oracle vs reference ok", {k: float(np.abs(v).mean()) for k, v in res.items() if v.dtype.kind == "f"})
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     ns = ref_shim.import_reference()
-    which = sys.argv[1:] or ["unet", "attention", "token_maps", "sd", "xl", "xl_labels"]
+    which = sys.argv[1:] or ["unet", "attention", "token_maps", "sd", "xl", "xl_labels", "oracle_vs_reference"]
     torch.set_num_threads(max(1, os.cpu_count() or 1))
     if "unet" in which: gen_unet(ns)
     if "attention" in which: gen_attention(ns)
@@ -334,6 +402,7 @@ def main():
     if "sd" in which: gen_sd_loops(ns)
     if "xl" in which: gen_xl_loops(ns)
     if "xl_labels" in which: gen_xl_labels(ns)
+    if "oracle_vs_reference" in which: gen_oracle_vs_reference(ns)
 
 
 if __name__ == "__main__":

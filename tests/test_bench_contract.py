@@ -77,6 +77,21 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_float32_npy(tmp_path):
+    import numpy as np
+    import torch
+    lat = torch.randn(1, 4, 8, 8).half()
+    bench.dump_outputs(str(tmp_path / "out"), {"latents": lat, "color_loss": torch.tensor([0.25])})
+    got = np.load(tmp_path / "out" / "latents.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, lat.float().numpy())
+    assert np.load(tmp_path / "out" / "color_loss.npy").tolist() == [0.25]
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
 def test_committed_bench_lines_carry_every_contract_key():
     """The JSON lines measured on the B200 boxes this round (profiles/r02_bench_*.json) against the keys the driver's
     contract lists: metric / value / unit / n_gpus / steps / warmup / ms_per_step / higher_is_better / scaling /
